@@ -9,6 +9,8 @@ One "step" = one batched call of the hot path over the whole workload (262 144 u
 GPU; 4096 distinct synthetic units tiled x64 on the device to bound host prep time).  `value` is measured with the
 compressed batch resident in HBM; `e2e` goes through swc_deflate_decompress_batch_host with pinned HOST buffers, i.e.
 host->device and device->host copies inside the timed region (the same 262 144 units).
+`--dump-outputs DIR` writes what the last timed step returned (result tables, a seeded sample of decoded units) as
+DIR/*.npy; the corpus is seeded, so the same flags give the same inputs and two builds can be compared output for output.
 Multi-GPU: units are independent, every rank decodes its own shard with no data-path collective (weak scaling);
 rank 0 owns the unit list and scatters byte-balanced shards over NCCL; `multi_gpu.legs` adds the gather / all-gather variants.
 """
@@ -83,6 +85,31 @@ def host_memory_budget():
         except (OSError, ValueError):
             pass
     return avail
+
+
+DUMP_TABLE_UNITS = 1 << 18     # result-table rows dumped: 4 float64 columns = 8 MiB
+DUMP_OUTPUT_UNITS = 192        # decoded units dumped as float32 rows: 48 MiB (56 MiB in all with the tables, under 64 MB)
+
+
+def dump_outputs(b, out_dir, seed=0):
+    """Writes what the last b.run() returned to its caller as .npy files: status, decoded length and consumed bits of every
+    unit (of a seeded sample of 2^18 units in larger batches; `units.npy` holds their indices), and the decoded bytes of a
+    seeded sample of 192 units (`output.npy`, one row of UNIT values per unit in `output_units.npy`, zero past the decoded
+    length).  The same seed and batch give the same sample, so two builds can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    st, ln, used = b.results()
+    rng = np.random.default_rng(seed)
+    n = b.n
+    rows = np.arange(n) if n <= DUMP_TABLE_UNITS else np.sort(rng.choice(n, DUMP_TABLE_UNITS, replace=False))
+    picks = np.sort(rng.choice(n, min(n, DUMP_OUTPUT_UNITS), replace=False))
+    out = np.zeros((len(picks), UNIT), dtype=np.float32)
+    for r, i in enumerate(picks):
+        o, m = int(b.h_out_off[i]), min(int(ln[i]), UNIT)
+        out[r, :m] = b.d_out[o:o + m].cpu().numpy()
+    arrays = {"units": rows, "status": st[rows], "out_len": ln[rows], "consumed_bits": used[rows], "output_units": picks}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
+    np.save(os.path.join(out_dir, "output.npy"), out)
 
 
 def read_peaks():
@@ -341,6 +368,8 @@ def run_product(args):
     if world > 1:
         dist.all_reduce(job, op=dist.ReduceOp.SUM)
     value = float(job[0].item()) / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(b, args.dump_outputs)
 
     # ---- SURVEY §8e legs: decode-only / + gather to rank 0 / + all-gather, on a sub-batch whose gathered size fits every GPU ----
     legs = None
@@ -512,6 +541,8 @@ def main():
     ap.add_argument("--no-legs", action="store_true")
     ap.add_argument("--leg-units", type=int, default=32768)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as DIR/*.npy "
+                                                          "(product arm, rank 0's units; see dump_outputs)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
