@@ -62,6 +62,8 @@ int32_t swc_deflate_decompress(const uint8_t *in, size_t in_len, size_t start_bi
                                uint8_t **out, size_t *out_len, size_t *consumed_bits);
 /* scratch the batched call needs for `out_capacity_total` bytes of output buffer */
 size_t  swc_deflate_batch_scratch_bytes(uint64_t n, uint64_t out_capacity_total);
+/* Device batch: every out_off[i] must be a multiple of 16 (the kernels store whole 8- and 16-byte words inside
+ * [out_off[i], out_off[i] + out_cap[i])); out_base itself must be 16-byte aligned. in_off may have any alignment. */
 int32_t swc_deflate_decompress_batch(const uint8_t *in_base, const uint64_t *in_off, const uint64_t *in_len,
                                      const uint8_t *start_bits /* n entries 0..7, or NULL */,
                                      uint8_t *out_base, const uint64_t *out_off, const uint64_t *out_cap,
@@ -87,7 +89,8 @@ int32_t swc_lz4_decompress(const uint8_t *in, size_t in_len, const uint8_t *dict
 int32_t swc_lz4_multi_decompress(const uint8_t *in, size_t in_len, const uint8_t *dict, size_t dict_len,
                                  int32_t has_dict_id, uint32_t dict_id,
                                  uint8_t **out, size_t *out_len, size_t **frame_ends, size_t *n_frames);
-/* raw blocks; dict (device pointer, may be NULL) is the prefix every block may reference (independent-block mode) */
+/* raw blocks; dict (device pointer, may be NULL) is the prefix every block may reference (independent-block mode).
+ * As for Deflate, every out_off[i] must be a multiple of 16 and out_base 16-byte aligned: the kernels store 16-byte words. */
 int32_t swc_lz4_block_decompress_batch(const uint8_t *in_base, const uint64_t *in_off, const uint64_t *in_len,
                                        const uint8_t *dict, uint64_t dict_len,
                                        uint8_t *out_base, const uint64_t *out_off, const uint64_t *out_cap,

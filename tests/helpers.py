@@ -33,27 +33,47 @@ def fixtures(prefix):
 class LsbBitWriter:
     """BitByteData.LsbBitWriter: bits fill each byte from bit 0 upward; numbers are written LSB first."""
 
+    # Whole bytes go to `out`; the < 8 pending bits sit in the integer `acc` (bit k of acc = stream bit nbits_done + k).
     def __init__(self):
-        self.bits = []
+        self.out = bytearray()
+        self.acc = 0
+        self.nacc = 0
+
+    def __len__(self):
+        """number of bits written so far"""
+        return len(self.out) * 8 + self.nacc
 
     def write_bits(self, bits):
-        self.bits.extend(bits)
+        for b in bits:
+            self.write_number(b & 1, 1)
 
     def write_number(self, value, count):
-        for i in range(count):
-            self.bits.append((value >> i) & 1)
+        self.acc |= (value & ((1 << count) - 1)) << self.nacc
+        self.nacc += count
+        if self.nacc >= 8:
+            k = self.nacc >> 3
+            self.out += (self.acc & ((1 << (8 * k)) - 1)).to_bytes(k, "little")
+            self.acc >>= 8 * k
+            self.nacc &= 7
 
-    def align(self):
-        while len(self.bits) % 8:
-            self.bits.append(0)
+    def write_bytes(self, data):
+        """bytes at the current bit position (a byte-aligned writer appends them as they are)"""
+        if self.nacc == 0:
+            self.out += data
+        else:
+            for byte in data:
+                self.write_number(byte, 8)
+
+    def align(self, fill=0):
+        """pad to a byte boundary with `fill` bits (0 or 1)"""
+        if self.nacc:
+            pad = 8 - self.nacc
+            self.write_number((1 << pad) - 1 if fill else 0, pad)
 
     @property
     def data(self):
         self.align()
-        out = bytearray()
-        for i in range(0, len(self.bits), 8):
-            out.append(sum(b << k for k, b in enumerate(self.bits[i:i + 8])))
-        return bytes(out)
+        return bytes(self.out)
 
 
 # literal round-trip vectors of the reference's compression tests (DeflateCompressionTests.swift:7-83,
